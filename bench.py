@@ -67,6 +67,8 @@ def parse_args():
     ap.add_argument("--no-full-unit", action="store_true", help="CPU arm: skip the one complete 576-hypothesis unit")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-torch-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (final poses and per-detection scores) as DIR/<name>.npy")
     a = ap.parse_args()
     a.render_size = tuple(int(v) for v in a.render_size.lower().split("x"))
     assert a.render_size in GFLOP, f"--render-size must be one of {sorted(GFLOP)}"
@@ -294,6 +296,28 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def host_outputs(final):
+    """What run_inference_pipeline hands its caller for one frame, as host arrays: every tensor of the final collection
+    and every numeric column of its infos (one row per detection), in float32 or float64."""
+    out = {}
+    for name, t in final.tensors.items():
+        a = t.detach().cpu().numpy()
+        out[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    for col in final.infos.columns:
+        v = final.infos[col].to_numpy()
+        if np.issubdtype(v.dtype, np.number) or v.dtype == np.bool_:
+            out[f"infos_{col}"] = v if v.dtype in (np.float32, np.float64) else v.astype(np.float64)
+    return out
+
+
+def write_outputs(outputs, out_dir: Path):
+    total = sum(a.nbytes for a in outputs.values())
+    assert total <= 64 << 20, f"{total} bytes of outputs exceed the 64 MB dump limit"
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 # ---------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------
@@ -352,9 +376,12 @@ def run_mpx_arm(args):
     def read_back(final):  # the step's result on the host
         return final.poses.cpu(), final.infos["pose_score"].values
 
+    last = [None]  # the final collection of the most recent step (for --dump-outputs)
+
     def step_device(e=None):
         obs, det = frame_device()
-        return (e or est).run_inference_pipeline(obs, detections=det, **kw)[0]
+        last[0] = (e or est).run_inference_pipeline(obs, detections=det, **kw)[0]
+        return last[0]
 
     def run_single(steps, host: bool):  # one blocking call per step
         for _ in range(steps):
@@ -370,10 +397,12 @@ def run_mpx_arm(args):
             done = pipe.submit(*(frame_host() if host else frame_device()), **kw)
             if done is not None:
                 n_done += 1
+                last[0] = done[0]
                 if host:
                     read_back(done[0])
         for done in pipe.drain():
             n_done += 1
+            last[0] = done[0]
             if host:
                 read_back(done[0])
         pipe.join()
@@ -406,6 +435,8 @@ def run_mpx_arm(args):
     if rank == 0:
         sampler.start()
     total_ms = timed(run, args.steps, False)
+    # copied out before later steps reuse the estimators' static buffers
+    outputs = host_outputs(last[0]) if args.dump_outputs else None
     run(2 * n_fif, True)
     e2e_ms = timed(run, args.steps, True)
     single = None
@@ -514,6 +545,8 @@ def run_mpx_arm(args):
                 line["gpu_torch_baseline"] = {"failed": repr(exc)[:300]}
         if n_gpus == 1 and not args.no_cpu_baseline and args.workload == "rgb576":
             line["cpu_baseline"] = cpu_baseline_subprocess(args)
+        if outputs is not None:
+            write_outputs(outputs, Path(args.dump_outputs))
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

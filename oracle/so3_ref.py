@@ -1,8 +1,7 @@
 """oracle/so3_ref.py -- SO(3) grid for the CPU oracle (TEST INFRASTRUCTURE ONLY).
 
-Restates load_SO3_grid (src/megapose/utils/transform_utils.py:27-50).  On machines with
-/root/reference the quaternions are parsed from the reference's own text file; elsewhere from the
-converted data asset (tests/test_oracle_vs_reference.py checks both agree).
+Restates load_SO3_grid (src/megapose/utils/transform_utils.py:27-50) on the converted data asset
+(tests/test_oracle_vs_reference.py holds the asset to the grid parsed from the reference's own text file).
 """
 from __future__ import annotations
 
@@ -13,15 +12,10 @@ import torch
 
 from .lib3d_ref import unitquat_to_rotmat
 
-_REF = Path("/root/reference/src/megapose/data")
 _ASSET = Path(__file__).resolve().parents[1] / "megapose6d_b200" / "data"
 
 
 def load_quats(resolution: int) -> torch.Tensor:
-    ref = _REF / f"data_{resolution}.qua"
-    if ref.is_file():
-        quats = [[float(v) for v in line.split()] for line in ref.read_text().splitlines() if line.strip()]
-        return torch.tensor(quats)
     return torch.tensor(np.load(_ASSET / f"so3_grid_{resolution}.npy").tolist())
 
 

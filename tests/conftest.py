@@ -10,16 +10,12 @@ if str(ROOT) not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (only present in the build container)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     has_gpu = torch.cuda.is_available()
-    has_ref = Path("/root/reference/src/megapose").is_dir()
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))

@@ -1,8 +1,10 @@
-"""Detector front-end (SURVEY 8 f4): the product's Detector against the reference's own class loaded by path
-(src/megapose/inference/detector.py:34-142), fed by the same stand-in network; load_detector round trip."""
+"""Detector front-end (SURVEY 8 f4): the product's Detector against what the reference's own class
+(src/megapose/inference/detector.py:34-142) returned when fed by the same stand-in network (tests/golden/detector.npz,
+written by `reference_outputs(ref)` through tools/make_golden.py); load_detector round trip."""
 import importlib.util
 import sys
 import types
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -11,7 +13,9 @@ import torch
 from megapose6d_b200 import detector as D
 from megapose6d_b200.load_model import Cfg
 from megapose6d_b200.types import ObservationTensor
-from oracle import refload
+from tests import helpers
+
+GOLDEN = Path(__file__).resolve().parent / "golden" / "detector.npz"
 
 
 class FakeMaskRCNN(torch.nn.Module):
@@ -34,8 +38,9 @@ class FakeMaskRCNN(torch.nn.Module):
         return out
 
 
-def _reference_detector_cls():
-    ref = refload.load()
+def _reference_detector_cls(ref):
+    from oracle import refload
+
     name = "megapose.inference.detector"
     if name not in sys.modules:
         sys.modules.setdefault("megapose.utils", types.ModuleType("megapose.utils")).tensor_collection = ref.tensor_collection
@@ -43,7 +48,7 @@ def _reference_detector_cls():
         mod = importlib.util.module_from_spec(spec)
         sys.modules[name] = mod
         spec.loader.exec_module(mod)
-    return sys.modules[name].Detector, ref
+    return sys.modules[name].Detector
 
 
 def _same(a, b):
@@ -64,21 +69,48 @@ def _same(a, b):
         assert torch.equal(a.masks.cpu(), b.masks.cpu())
 
 
-@pytest.mark.skipif(not refload.available(), reason="needs /root/reference")
-@pytest.mark.parametrize("counts", [(3, 0, 5), (1,), (4, 4)])
-@pytest.mark.parametrize("kw", [dict(), dict(detection_th=0.4), dict(output_masks=True, mask_th=0.6),
-                                dict(one_instance_per_class=True, detection_th=0.1, output_masks=True)])
-def test_detector_matches_reference_class(counts, kw):
-    RefDetector, ref = _reference_detector_cls()
-    images = torch.rand(len(counts), 3, 24, 32)
-    K = torch.eye(3).repeat(len(counts), 1, 1)
+COUNTS = [(3, 0, 5), (1,), (4, 4)]
+KWS = [dict(), dict(detection_th=0.4), dict(output_masks=True, mask_th=0.6),
+       dict(one_instance_per_class=True, detection_th=0.1, output_masks=True)]
+
+
+def _detector_inputs(counts):
+    return torch.rand(len(counts), 3, 24, 32), torch.eye(3).repeat(len(counts), 1, 1)
+
+
+def _rgb():
+    return (np.random.RandomState(0).rand(24, 32, 3) * 255).astype(np.uint8)
+
+
+@pytest.fixture(scope="module")
+def want():
+    return np.load(GOLDEN)
+
+
+@pytest.mark.parametrize("counts", COUNTS)
+@pytest.mark.parametrize("kw", KWS)
+def test_detector_matches_reference_class(want, counts, kw):
+    images, K = _detector_inputs(counts)
     mine = D.Detector(FakeMaskRCNN(counts))
     got = mine.get_detections(ObservationTensor(images, K), **kw)
-    with refload.cpu_cuda_patch():
-        want = RefDetector(FakeMaskRCNN(counts)).get_detections(ref.types.ObservationTensor(images, K), **kw)
-    _same(got, want)
-    rgb = (np.random.RandomState(0).rand(24, 32, 3) * 255).astype(np.uint8)
-    assert torch.equal(mine.image_tensor_from_numpy(rgb), RefDetector(FakeMaskRCNN(counts)).image_tensor_from_numpy(rgb))
+    _same(got, helpers.restore_collection(want, f"{COUNTS.index(counts)}/{KWS.index(kw)}"))
+    assert helpers.tensor_digest(mine.image_tensor_from_numpy(_rgb())) == str(want["image_tensor"])
+
+
+def reference_outputs(ref) -> dict:
+    """What the reference's Detector returns on the inputs of test_detector_matches_reference_class (tools/make_golden.py)."""
+    from oracle import refload
+
+    RefDetector = _reference_detector_cls(ref)
+    out = {}
+    for i, counts in enumerate(COUNTS):
+        for j, kw in enumerate(KWS):
+            images, K = _detector_inputs(counts)
+            with refload.cpu_cuda_patch():
+                a = RefDetector(FakeMaskRCNN(counts)).get_detections(ref.types.ObservationTensor(images, K), **kw)
+            helpers.record_collection(out, f"{i}/{j}", a)
+    out["image_tensor"] = np.array(helpers.tensor_digest(RefDetector(FakeMaskRCNN((1,))).image_tensor_from_numpy(_rgb())))
+    return out
 
 
 def test_detector_without_detections():

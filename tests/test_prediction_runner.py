@@ -1,14 +1,17 @@
-"""Frame-level caller (megapose6d_b200/prediction_runner.py): host logic on the CPU with a stand-in estimator, the REAL
-reference caller (loaded by path, marker `reference`) as the checker, and a world_size-2 gloo run of the frame sharding.
+"""Frame-level caller (megapose6d_b200/prediction_runner.py): host logic on the CPU with a stand-in estimator, what the
+REAL reference caller returned on the same frames as the checker (tests/golden/prediction_runner.npz, written by
+`reference_outputs(ref)` through tools/make_golden.py), and a world_size-2 gloo run of the frame sharding.
 
 The stand-in estimator is a deterministic function of the observation and the detections; it works with the reference's
 collections and with ours, so the reference's `PredictionRunner` and ours can be driven by the same object."""
 import importlib.util
+import json
 import os
 import pickle
 import socket
 import sys
 import types
+from pathlib import Path
 
 import numpy as np
 import pandas as pd
@@ -20,6 +23,7 @@ import torch.multiprocessing as mp
 from megapose6d_b200 import prediction_runner as pr
 from megapose6d_b200.example import CameraData, ObjectData
 from megapose6d_b200.types import InferenceConfig
+from tests import helpers
 
 
 # ------------------------------------------------------------------------------------------------------ fixtures
@@ -103,14 +107,82 @@ def _same_collection(a, b, drop=("time",)):
 
 
 # ------------------------------------------------------------------------------------------- the reference's caller
+GOLDEN = Path(__file__).resolve().parent / "golden" / "prediction_runner.npz"
+SAMPLER_CASES = [(n, world, shuffle, rank) for n in (1, 2, 7, 50, 1000) for world in (1, 2, 3, 8) for shuffle in (True, False)
+                 for rank in range(world)]
+COLLATE_LABELS = (None, ["obj_000001", "obj_000002", "obj_000003"])
+RUNNER_MODES = ("gt", "external", "depth_refiner")
+
+
 @pytest.fixture(scope="module")
-def ref_caller():
+def want():
+    return np.load(GOLDEN)
+
+
+def _runner_cfg(mode):
+    return InferenceConfig(**{**CFG.__dict__, **dict(coarse_estimation_type="external" if mode == "external" else "SO3_grid",
+                                                     run_depth_refiner=(mode == "depth_refiner"))})
+
+
+def test_sampler_matches_the_reference(want):
+    state = np.random.get_state()[1].copy()
+    ends = np.cumsum(want["sampler/lengths"])
+    for k, (n, world, shuffle, rank) in enumerate(SAMPLER_CASES):
+        b = pr.DistributedSceneSampler(range(n), world, rank, shuffle=shuffle)
+        w = want["sampler/indices"][ends[k] - want["sampler/lengths"][k]:ends[k]]
+        assert list(b) == w.tolist() and len(b) == len(w)
+    assert np.array_equal(state, np.random.get_state()[1])
+
+
+@pytest.mark.parametrize("with_init", [False, True])
+def test_collate_matches_the_reference(want, with_init):
+    obs = make_observations(3, with_init=with_init)
+    for n_labels, labels in enumerate(COLLATE_LABELS):
+        p = f"collate/{with_init}/{n_labels}"
+        b = pr.SceneObservation.collate_fn(obs, labels)
+        assert sorted(b) == sorted(str(k) for k in want[f"{p}/keys"])
+        assert helpers.tensor_digest(b["rgb"]) == str(want[f"{p}/rgb"]) and helpers.tensor_digest(b["depth"]) == str(want[f"{p}/depth"])
+        assert json.loads(str(want[f"{p}/im_infos"])) == b["im_infos"]
+        assert torch.equal(torch.from_numpy(want[f"{p}/K"]), b["cameras"].K)
+        for k in ("gt_detections", "gt_data", "initial_data"):
+            if f"{p}/{k}/tensors" not in want:
+                assert b[k] is None
+            else:
+                _same_collection(helpers.restore_collection(want, f"{p}/{k}"), b[k])
+                assert b[k].poses.dtype == torch.float32
+
+
+@pytest.mark.parametrize("mode", RUNNER_MODES)
+def test_runner_matches_the_reference_runner(want, mode):
+    """Same frames, same stand-in estimator, the reference's PredictionRunner against ours: per-key predictions equal (but
+    for our extra `time` column), same frame order, the first frame run twice (warm-up) by both."""
+    obs = make_observations(5, with_init=(mode == "external"))
+    runner = pr.PredictionRunner(pr.ListSceneDataset(obs, load_depth=True), _runner_cfg(mode), device="cpu")
+    est_b = StandInEstimator()
+    got = runner.get_predictions(est_b)
+    p = f"runner/{mode}"
+    assert json.loads(json.dumps([list(c) for c in est_b.calls])) == json.loads(str(want[f"{p}/calls"])) and len(est_b.calls) == len(obs) + 1
+    assert set(got) == {str(k) for k in want[f"{p}/keys"]}
+    for k in got:
+        _same_collection(helpers.restore_collection(want, f"{p}/{k}"), got[k])
+        assert "time" in got[k].infos
+    assert [(t["scene_id"], t["view_id"]) for t in runner.frame_times] == \
+        [(obs[i].infos.scene_id, obs[i].infos.view_id) for i in runner.sampler]
+
+
+def test_bop_csv_matches_the_toolkit_writer(tmp_path, want):
+    """Byte-for-byte against the BOP toolkit's `inout.save_bop_results` as vendored by the reference."""
+    pr.save_bop_results(tmp_path / "mine.csv", pr.predictions_to_bop(_predictions(7)))
+    assert (tmp_path / "mine.csv").read_bytes() == want["bop_csv"].tobytes()
+
+
+def _reference_caller(ref):
     """The reference's samplers.py, scene_dataset.py and prediction_runner.py, loaded by path on top of oracle/refload.py.
     Stubbed (absent packages): webdataset, pinocchio's Transform (a numpy 4x4 holder: the runner only reads `.matrix`),
     megapose.utils.random (its two pure-Python helpers are exec'ed from the source), DataLoader workers (n_workers=0)."""
     from oracle import refload
 
-    ns = refload.load()
+    ns = ref
     ref_root = refload.REF_ROOT
     sys.modules.setdefault("webdataset", types.ModuleType("webdataset"))
 
@@ -170,93 +242,77 @@ def _to_reference_observation(ref_caller, obs):
                               object_datas=objs, camera_data=cam)
 
 
-@pytest.mark.reference
-def test_sampler_matches_the_reference(ref_caller):
+def reference_outputs(ref) -> dict:
+    """What the reference's caller returns on the inputs of the tests above (tools/make_golden.py -> GOLDEN)."""
+    from oracle import refload
+
+    R = _reference_caller(ref)
+    out = {}
     state = np.random.get_state()[1].copy()
-    for n in (1, 2, 7, 50, 1000):
-        for world in (1, 2, 3, 8):
-            for shuffle in (True, False):
-                for rank in range(world):
-                    a = ref_caller.samplers.DistributedSceneSampler(range(n), world, rank, shuffle=shuffle)
-                    b = pr.DistributedSceneSampler(range(n), world, rank, shuffle=shuffle)
-                    assert list(a) == list(b) and len(a) == len(b)
+    lists = []
+    for n, world, shuffle, rank in SAMPLER_CASES:
+        a = R.samplers.DistributedSceneSampler(range(n), world, rank, shuffle=shuffle)
+        assert len(a) == len(list(a))
+        lists.append(list(a))
+    out["sampler/lengths"] = np.array([len(x) for x in lists], dtype=np.int32)
+    out["sampler/indices"] = np.concatenate([np.asarray(x, dtype=np.int32) for x in lists])
     assert np.array_equal(state, np.random.get_state()[1])
 
+    for with_init in (False, True):
+        obs = make_observations(3, with_init=with_init)
+        for n_labels, labels in enumerate(COLLATE_LABELS):
+            p = f"collate/{with_init}/{n_labels}"
+            a = R.scene_dataset.SceneObservation.collate_fn([_to_reference_observation(R, o) for o in obs], labels)
+            out[f"{p}/keys"] = np.array(sorted(a), dtype="U")
+            out[f"{p}/rgb"], out[f"{p}/depth"] = np.array(helpers.tensor_digest(a["rgb"])), np.array(helpers.tensor_digest(a["depth"]))
+            out[f"{p}/K"] = a["cameras"].K.numpy()
+            out[f"{p}/im_infos"] = np.array(json.dumps(a["im_infos"]))
+            for k in ("gt_detections", "gt_data", "initial_data"):
+                if a[k] is not None:
+                    helpers.record_collection(out, f"{p}/{k}", a[k])
 
-@pytest.mark.reference
-@pytest.mark.parametrize("with_init", [False, True])
-def test_collate_matches_the_reference(ref_caller, with_init):
-    obs = make_observations(3, with_init=with_init)
-    for labels in (None, ["obj_000001", "obj_000002", "obj_000003"]):
-        a = ref_caller.scene_dataset.SceneObservation.collate_fn([_to_reference_observation(ref_caller, o) for o in obs], labels)
-        b = pr.SceneObservation.collate_fn(obs, labels)
-        assert set(a) == set(b)
-        assert torch.equal(a["rgb"], b["rgb"]) and torch.equal(a["depth"], b["depth"])
-        assert a["im_infos"] == b["im_infos"]
-        assert torch.equal(a["cameras"].K, b["cameras"].K)
-        for k in ("gt_detections", "gt_data", "initial_data"):
-            if a[k] is None:
-                assert b[k] is None
-            else:
-                _same_collection(a[k], b[k])
-                assert a[k].poses.dtype == b[k].poses.dtype == torch.float32
+    # device moves of the reference (hard-coded .cuda()) -> identity on the host
+    TC, Obs = R.ns.tensor_collection.TensorCollection, R.ns.types.ObservationTensor
+    U = sys.modules["megapose.inference.utils"]
+    saved = (TC.cuda, Obs.cuda, U.add_instance_id)
+    TC.cuda, Obs.cuda = (lambda self: self), (lambda self, *a: self)
+    try:
+        for mode in RUNNER_MODES:
+            obs = make_observations(5, with_init=(mode == "external"))
 
+            class RefDataset(R.scene_dataset.SceneDataset):
+                def __init__(self):
+                    super().__init__(pd.DataFrame(dict(scene_id=[o.infos.scene_id for o in obs],
+                                                       view_id=[o.infos.view_id for o in obs])), load_depth=True)
 
-@pytest.mark.reference
-@pytest.mark.parametrize("mode", ["gt", "external", "depth_refiner"])
-def test_runner_matches_the_reference_runner(ref_caller, mode, monkeypatch):
-    """Same frames, same stand-in estimator, the reference's PredictionRunner against ours: per-key predictions equal (but
-    for our extra `time` column), same frame order, the first frame run twice (warm-up) by both."""
-    obs = make_observations(5, with_init=(mode == "external"))
-    cfg = InferenceConfig(**{**CFG.__dict__, **dict(coarse_estimation_type="external" if mode == "external" else "SO3_grid",
-                                                    run_depth_refiner=(mode == "depth_refiner"))})
-    R = ref_caller
+                def _load_scene_observation(self, infos):
+                    o = next(o for o in obs if (o.infos.scene_id, o.infos.view_id) == (infos.scene_id, infos.view_id))
+                    return _to_reference_observation(R, o)
 
-    class RefDataset(R.scene_dataset.SceneDataset):
-        def __init__(self):
-            super().__init__(pd.DataFrame(dict(scene_id=[o.infos.scene_id for o in obs], view_id=[o.infos.view_id for o in obs])),
-                             load_depth=True)
+            U.add_instance_id = saved[2]
+            if mode == "external":
+                # the reference helper relies on groupby().apply() keeping the grouping columns (true for the pandas it pins,
+                # not for the one used here, see tests/test_product_vs_reference.py): put them back after its own call
+                def add_instance_id(inputs, original=saved[2]):
+                    before = inputs.infos[["batch_im_id", "label"]].copy()
+                    res = original(inputs)
+                    for c in before:
+                        if c not in res.infos:
+                            res.infos[c] = before[c]
+                    return res
 
-        def _load_scene_observation(self, infos):
-            o = next(o for o in obs if (o.infos.scene_id, o.infos.view_id) == (infos.scene_id, infos.view_id))
-            return _to_reference_observation(R, o)
+                U.add_instance_id = add_instance_id
+            runner = R.prediction_runner.PredictionRunner(RefDataset(), R.ns.types.InferenceConfig(**_runner_cfg(mode).__dict__),
+                                                          batch_size=1, n_workers=0)
+            est = StandInEstimator()
+            preds = runner.get_predictions(est)
+            out[f"runner/{mode}/calls"] = np.array(json.dumps([list(c) for c in est.calls]))
+            out[f"runner/{mode}/keys"] = np.array(sorted(preds), dtype="U")
+            for k, v in preds.items():
+                helpers.record_collection(out, f"runner/{mode}/{k}", v)
+    finally:
+        TC.cuda, Obs.cuda, U.add_instance_id = saved
 
-    # device moves of the reference (hard-coded .cuda()) -> identity on this CPU-only machine
-    monkeypatch.setattr(R.ns.tensor_collection.TensorCollection, "cuda", lambda self: self)
-    monkeypatch.setattr(R.ns.types.ObservationTensor, "cuda", lambda self, *a: self)
-    if mode == "external":
-        # the reference helper relies on groupby().apply() keeping the grouping columns (true for the pandas it pins, not for
-        # the one installed here, see tests/test_product_vs_reference.py): put them back after the reference's own call
-        U = sys.modules["megapose.inference.utils"]
-        original = U.add_instance_id
-
-        def add_instance_id(inputs):
-            before = inputs.infos[["batch_im_id", "label"]].copy()
-            out = original(inputs)
-            for c in before:
-                if c not in out.infos:
-                    out.infos[c] = before[c]
-            return out
-
-        monkeypatch.setattr(U, "add_instance_id", add_instance_id)
-    ref_cfg = R.ns.types.InferenceConfig(**cfg.__dict__)
-    ref_runner = R.prediction_runner.PredictionRunner(RefDataset(), ref_cfg, batch_size=1, n_workers=0)
-    est_a, est_b = StandInEstimator(), StandInEstimator()
-    want = ref_runner.get_predictions(est_a)
-    runner = pr.PredictionRunner(pr.ListSceneDataset(obs, load_depth=True), cfg, device="cpu")
-    got = runner.get_predictions(est_b)
-    assert est_a.calls == est_b.calls and len(est_b.calls) == len(obs) + 1
-    assert set(want) == set(got)
-    for k in want:
-        _same_collection(want[k], got[k])
-        assert "time" in got[k].infos
-    assert [(t["scene_id"], t["view_id"]) for t in runner.frame_times] == \
-        [(obs[i].infos.scene_id, obs[i].infos.view_id) for i in runner.sampler]
-
-
-@pytest.mark.reference
-def test_bop_csv_matches_the_toolkit_writer(tmp_path):
-    """Byte-for-byte against the BOP toolkit's `inout.save_bop_results` as vendored by the reference."""
     for name in ("imageio", "png"):
         sys.modules.setdefault(name, types.ModuleType(name))
     pkg = types.ModuleType("bop_toolkit_lib")
@@ -265,14 +321,15 @@ def test_bop_csv_matches_the_toolkit_writer(tmp_path):
     sys.modules.setdefault("bop_toolkit_lib", pkg)
     sys.modules.setdefault("bop_toolkit_lib.misc", pkg.misc)
     spec = importlib.util.spec_from_file_location(
-        "bop_toolkit_lib_inout_ref", "/root/reference/deps/bop_toolkit_challenge/bop_toolkit_lib/inout.py")
+        "bop_toolkit_lib_inout_ref", refload.REF_ROOT.parents[1] / "deps/bop_toolkit_challenge/bop_toolkit_lib/inout.py")
     inout = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(inout)
-    preds = _predictions(7)
-    rows = pr.predictions_to_bop(preds)
-    inout.save_bop_results(str(tmp_path / "ref.csv"), rows)
-    pr.save_bop_results(tmp_path / "mine.csv", rows)
-    assert (tmp_path / "ref.csv").read_bytes() == (tmp_path / "mine.csv").read_bytes()
+    import tempfile
+
+    with tempfile.TemporaryDirectory() as tmp:
+        inout.save_bop_results(str(Path(tmp) / "ref.csv"), pr.predictions_to_bop(_predictions(7)))
+        out["bop_csv"] = np.frombuffer((Path(tmp) / "ref.csv").read_bytes(), dtype=np.uint8)
+    return out
 
 
 # ------------------------------------------------------------------------------------------ no reference needed

@@ -155,8 +155,25 @@ def fullsize_fixture(ref, name: str):
     print(f"{name}: {n_det} detections x {sc['grid']} hypotheses, {time.time() - t0:.1f} s on {threads} threads", flush=True)
 
 
+REFERENCE_TEST_MODULES = ("test_oracle_vs_reference", "test_product_vs_reference", "test_prediction_runner", "test_detector")
+
+
+def reference_test_fixtures(ref, modules=REFERENCE_TEST_MODULES):
+    """tests/golden/<module without test_>.npz: what the reference returned on the inputs of each module's comparisons
+    with the reference (computed by the module's own `reference_outputs(ref)`)."""
+    import importlib
+
+    for name in modules:
+        arrays = importlib.import_module(f"tests.{name}").reference_outputs(ref)
+        path = OUT / f"{name[len('test_'):]}.npz"
+        np.savez_compressed(path, **arrays)
+        print(f"{path.name}: {len(arrays)} arrays, {path.stat().st_size} bytes", flush=True)
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1:  # python tools/make_golden.py fullsize_rgb fullsize_rgb_224 ...
+    if sys.argv[1:2] == ["tests"]:  # python tools/make_golden.py tests [test_module ...]
+        reference_test_fixtures(refload.load(), sys.argv[2:] or REFERENCE_TEST_MODULES)
+    elif len(sys.argv) > 1:  # python tools/make_golden.py fullsize_rgb fullsize_rgb_224 ...
         _ref = refload.load()
         for _name in sys.argv[1:]:
             fullsize_fixture(_ref, _name)
