@@ -88,7 +88,9 @@ int mpx_meshdb_set_textures(mpx_meshdb* db, const float* h_uv, const uint8_t* h_
                                       * axes at 10 bounding radii, panda3d_scene_renderer.py:104-136) instead of ambient 1.0:
                                       * what models with render_normals=False are fed (models/pose_rigid.py:374-378) */
 /* depth normalisation of the fused depth channels (PosePredictor.normalize_depth, models/pose_rigid.py:466-496), applied
- * with d_depth_norm_z[sample] = tCR_z; raster entry points carry it in flags bits 8-9, mpx_roi_align_fused as an argument */
+ * with d_depth_norm_z[sample] = tCR_z; raster entry points carry it in flags bits 8-9, mpx_roi_align_fused as an argument.
+ * NaN follows torch.clamp: a NaN depth / z or depth - z (0 / 0 on the background when z == 0, a NaN z) stays NaN through
+ * the clamps, and the network input receives NaN. */
 #define MPX_DEPTH_NORM_TCR_SCALE_CLAMP_CENTER 0  /* clamp(depth / z, 0, 2) - 1 (the released RGB-D refiner) */
 #define MPX_DEPTH_NORM_TCR_SCALE 1               /* depth / z */
 #define MPX_DEPTH_NORM_TCR_CENTER_CLAMP 2        /* clamp(depth - z, -2, 2) */

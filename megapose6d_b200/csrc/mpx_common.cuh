@@ -118,11 +118,19 @@ __device__ __forceinline__ act_t to_act(float v) {
 #endif
 
 // depth normalisation of PosePredictor.normalize_depth (models/pose_rigid.py:466-496); kind as in include/mpx.h
-// (MPX_DEPTH_NORM_*): 0 tCR_scale_clamp_center, 1 tCR_scale, 2 tCR_center_clamp, 3 none
+// (MPX_DEPTH_NORM_*): 0 tCR_scale_clamp_center, 1 tCR_scale, 2 tCR_center_clamp, 3 none.  A NaN quotient / difference
+// (0 / 0 on the background when z == 0, or a NaN z) passes through as torch.clamp lets it; fminf / fmaxf alone would
+// return the bound instead.
 __device__ __forceinline__ float depth_norm(float d, float z, int kind) {
-  if (kind == 0) return fminf(fmaxf(__fdiv_rn(d, z), 0.f), 2.f) - 1.f;
+  if (kind == 0) {
+    const float q = __fdiv_rn(d, z);
+    return q != q ? q : fminf(fmaxf(q, 0.f), 2.f) - 1.f;
+  }
   if (kind == 1) return __fdiv_rn(d, z);
-  if (kind == 2) return fminf(fmaxf(d - z, -2.f), 2.f);
+  if (kind == 2) {
+    const float q = d - z;
+    return q != q ? q : fminf(fmaxf(q, -2.f), 2.f);
+  }
   return d;
 }
 
